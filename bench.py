@@ -248,17 +248,22 @@ def cpu_leg_cfg3(g, nlines: int, threads: int, full_at: int | None = None):
 
 def cpu_leg_stream(fsm, text: np.ndarray):
     """One reference fsm_exec call over `text` (serial by nature), as-is; amortised = the reference's
-    own per-byte transition without the per-call validation."""
+    own per-byte transition without the per-call validation.  Without the compiled reference, the
+    oracle's port of the same walk (kind "port"), as in the config-2 leg."""
     import reflib
-    assert reflib.have_ref()
-    R = reflib.Ref(); h = R.from_flat(fsm)
-    t0 = time.perf_counter(); rc, end, consumed = R.exec(h, text.tobytes()); dt0 = time.perf_counter() - t0
     off = np.array([0, text.size], dtype=np.uint64)
-    t0 = time.perf_counter(); rec = R.exec_batch(h, text, off, mode=1, nthreads=1); dt1 = time.perf_counter() - t0
-    R.free(h)
+    if reflib.have_ref():
+        R = reflib.Ref(); h = R.from_flat(fsm); kind = "reference"
+        t0 = time.perf_counter(); rc, end, consumed = R.exec(h, text.tobytes()); dt0 = time.perf_counter() - t0
+        t0 = time.perf_counter(); R.exec_batch(h, text, off, mode=1, nthreads=1); dt1 = time.perf_counter() - t0
+        R.free(h)
+    else:
+        O = reflib.Oracle(); kind = "port"
+        t0 = time.perf_counter(); rc, end, consumed = O.exec(fsm, text.tobytes()); dt0 = time.perf_counter() - t0
+        t0 = time.perf_counter(); O.exec_batch(fsm, text, off); dt1 = time.perf_counter() - t0
     g0, g1 = text.size / dt0 / 1e9, text.size / dt1 / 1e9
     return {"asis_gbs": g0, "asis_threads": 1, "asis_s": dt0, "amortised_gbs": g1, "amortised_threads": 1,
-            "asis_1t_gbs": g0, "amortised_1t_gbs": g1, "threads_swept": [1], "kind": "reference",
+            "asis_1t_gbs": g0, "amortised_1t_gbs": g1, "threads_swept": [1], "kind": kind,
             "record": (int(rc), int(end), int(consumed))}
 
 
@@ -577,6 +582,15 @@ def run_cfg2(args):
             assert torch.equal(mine, d_out[0]), "bench: all-gather slot mismatch"
 
     ms_total, launches, sampler = timed_region(c, step, args.steps, args.warmup)
+    if args.dump_outputs is not None and rank == 0:
+        last = (step_no[0] - 1) % nbuf                    # the buffer the last timed step wrote
+        if fused and compact:
+            recs = L.results_from_torch(own_out[last])
+        elif fused:
+            recs = ring.read(last)[rank * n:(rank + 1) * n]
+        else:
+            recs = L.results_from_torch(d_out[last])
+        dump_outputs(args.dump_outputs, record_fields(recs))
 
     def one_kernel(inp=d_in):
         if fused:
@@ -651,6 +665,44 @@ def run_cfg2(args):
         if ring is not None:
             ring.close()
     return finish(c)
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """--dump-outputs: each array as DIR/<name>.npy in float64, which holds every value written here exactly
+    (integers below 2^53: 64-bit bitsets are split into 32-bit words first)."""
+    out = {name: np.asarray(a).astype(np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the 64 MiB limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
+def record_fields(recs: np.ndarray) -> dict:
+    """The fields of result records (ret, end, consumed) as separate arrays."""
+    return {name: recs[name] for name in recs.dtype.names}
+
+
+def dense_rows(f, states: np.ndarray) -> np.ndarray:
+    """Rows [len(states), 256] of f's dense transition table (0xFFFFFFFF = no edge; the first group that
+    holds a symbol wins, as in FlatFsm.dense_table), computed for the given states only."""
+    rows = np.full((len(states), 256), 0xFFFFFFFF, dtype=np.uint32)
+    for k, s in enumerate(states):
+        lo, hi = int(f.group_off[s]), int(f.group_off[s + 1])
+        bits = np.unpackbits(np.ascontiguousarray(f.group_symbols[lo:hi], dtype="<u8").view(np.uint8).reshape(hi - lo, 32),
+                             axis=1, bitorder="little").astype(bool)
+        for g in range(hi - lo - 1, -1, -1):
+            rows[k, bits[g]] = f.group_to[lo + g]
+    return rows
+
+
+def u32_words(a) -> np.ndarray:
+    """64-bit words as pairs of 32-bit words (low first), exact in float64."""
+    return np.ascontiguousarray(a).view(np.uint64).view(np.uint32).reshape(len(a), -1)
 
 
 def bind_to_gpu_numa(local: int):
@@ -730,6 +782,12 @@ def run_cfg3(args):
     assert (masks[:ns].cpu().numpy().view(np.uint64) == wmasks).all(), "bench: config 3 fired-id sets differ from the reference"
 
     ms_total, launches, sampler = timed_region(c, step, args.steps, args.warmup)
+    if args.dump_outputs is not None and rank == 0:
+        # 10 M lines of records + bitsets exceed 64 MiB: a fixed sample of 2^19 lines (seed 0), their indices included
+        pick = np.sort(np.random.default_rng(0).choice(nlines, size=min(nlines, 1 << 19), replace=False))
+        tpick = torch.from_numpy(pick).to(dev)
+        dump_outputs(args.dump_outputs, {"line": pick, **record_fields(L.results_from_torch(rec[tpick])),
+                                         "fired_words": u32_words(masks[tpick].cpu().numpy())})
     kms = kernel_ms(c, launch, args.steps)
     clocks = sampler.finish()
 
@@ -887,9 +945,13 @@ def run_cfg4(args):
         R.free(h)
         assert (rc, rcons) == dfa.exec_stream(shard[:cut])[0::2], "bench: config 4 differs from the reference on the prefix"
 
+    last = [None]
+
     def step(_i):
-        scan(shard)
+        last[0] = scan(shard)
     ms_total, launches, sampler = timed_region(c, step, args.steps, args.warmup)
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("ret", "end", "consumed"), ([v] for v in last[0]))))
     # the body kernel's share: exec_stream is a handful of launches; time the whole device-side call
     t = []
     for _ in range(max(3, min(args.steps, 10))):
@@ -955,10 +1017,14 @@ def run_cfg1(args):
     want = oracle.exec(fsm, text.tobytes(), validate=False)
     assert dfa.exec_stream(d_text) == want, "bench: config 1 differs from the oracle"
 
+    last = [None]
+
     def step(_i):
         flush.fill_(1)                               # input smaller than L2: evict it between iterations
-        dfa.exec_stream(d_text)
+        last[0] = dfa.exec_stream(d_text)
     ms_total, launches, sampler = timed_region(c, step, args.steps, args.warmup)
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("ret", "end", "consumed"), ([v] for v in last[0]))))
     tt = []
     for _ in range(max(5, min(args.steps, 20))):
         flush.fill_(1)
@@ -1038,6 +1104,12 @@ def run_cfg5(args):
         if i >= args.warmup:
             times.append(s["ms_total"]); walls.append(w * 1e3)
         assert d.nstates == dfa.nstates
+    if args.dump_outputs is not None and rank == 0:
+        # the whole DFA (2.6 M label groups) exceeds 64 MiB: every state's end bit and end-id count, and the
+        # dense-table rows of a fixed sample of 8192 states (seed 0) with their indices
+        pick = np.sort(np.random.default_rng(0).choice(d.nstates, size=min(d.nstates, 8192), replace=False))
+        dump_outputs(args.dump_outputs, {"is_end": d.is_end, "endid_count": np.diff(d.endid_off), "state": pick,
+                                         "table_rows": dense_rows(d, pick)})
     sampler = ClockSampler(local); sampler.start(); clocks = sampler.finish()
     ms, wall = float(np.mean(times)), float(np.mean(walls))
     ms, wall = reduce_max(c, [ms, wall])
@@ -1086,7 +1158,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--config", type=int, default=2, choices=[1, 2, 3, 4, 5])
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 50; configs 3-5 of the GPU arm: 10)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--dist", default="uniform", choices=["uniform", "adversarial"])
@@ -1102,12 +1174,22 @@ def main():
     ap.add_argument("--gather", default="fused", choices=["fused", "nccl"],
                     help="N>1: fused = scanning lanes store records into every peer's buffer over NVLink P2P; "
                          "nccl = one NCCL all-gather per step on a side stream")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="GPU arm: after the timed steps, write what the last one computed to DIR/<name>.npy (float64): "
+                         "config 2 the result records, config 3 those of a fixed sample of 2^19 lines with their fired-id "
+                         "bitsets, configs 1 and 4 the one record of the stream, config 5 the end bits of the DFA and the table rows of "
+                         "a fixed sample of 8192 states; at N > 1, rank 0's shard")
     args = ap.parse_args()
+    if args.steps is None:
+        # seconds-long GPU setups: keep the default run within minutes
+        args.steps = 10 if args.config in (3, 4, 5) and args.impl == "b200" else 50
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs is for the GPU arm")
     if args.impl == "reference":
         return run_reference_arm(args)
     args.warmup = max(args.warmup, 3)
-    if args.config in (3, 4, 5) and args.steps == 50:
-        args.steps = 10                                   # seconds-long setups: keep the default run within minutes
     return {1: run_cfg1, 2: run_cfg2, 3: run_cfg3, 4: run_cfg4, 5: run_cfg5}[args.config](args)
 
 

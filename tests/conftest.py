@@ -10,7 +10,7 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a real B200 (run with -m gpu on the GPU box)")
-    config.addinivalue_line("markers", "needs_ref: needs oracle/_ref/libref_harness.so (the compiled reference)")
+    config.addinivalue_line("markers", "needs_ref: compares with the reference (live, or its recorded answers)")
 
 
 @pytest.fixture(scope="session")
@@ -22,6 +22,4 @@ def oracle():
 @pytest.fixture(scope="session")
 def ref():
     import reflib
-    if not reflib.have_ref():
-        pytest.skip("compiled reference (oracle/_ref/libref_harness.so) not available")
-    return reflib.Ref()
+    return reflib.reference()

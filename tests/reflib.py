@@ -2,14 +2,20 @@
 
   Oracle  oracle/_ref/libfsm_oracle.so   plain-C restatement (oracle/fsm_oracle.c)
   Ref     oracle/_ref/libref_harness.so  the unmodified reference compiled from
-                                         /root/reference (oracle/ref_harness.c)
+                                         its sources (oracle/ref_harness.c)
 
-Both are built by `make -C oracle`.  The prebuilt .so files travel to the GPU box;
-/root/reference itself is never read at test time.
+Both are built by `make -C oracle`, the harness only where the reference's sources are
+present; elsewhere RecordedRef answers with what the harness recorded.  The reference's
+sources are never read at test time.
 """
 from __future__ import annotations
 
+import atexit
+import base64
 import ctypes as C
+import hashlib
+import json
+import lzma
 import os
 import subprocess
 import sys
@@ -30,7 +36,7 @@ RE_LIKE, RE_LITERAL, RE_GLOB, RE_NATIVE, RE_SQL, RE_PCRE = range(6)
 
 
 def build_oracle() -> None:
-    """(Re)build the checkers; builds the reference too when /root/reference exists."""
+    """(Re)build the checkers; builds the reference too when its sources are present."""
     subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "-j8"], check=True,
                    stdout=subprocess.DEVNULL)
 
@@ -214,7 +220,37 @@ class RefFlat(C.Structure):
     _fields_ = [("desc", CDesc), ("blocks", C.c_void_p * 8)]
 
 
-class Ref:
+class _Recipes:
+    """Constructions built from the primitives, shared by Ref and RecordedRef."""
+
+    def compile_dfa(self, pattern, dialect: int = RE_PCRE, flags: int = 0, minimise: bool = True,
+                    endid: int | None = None):
+        """re_comp -> fsm_determinise [-> fsm_minimise] [-> fsm_setendid]; returns handle."""
+        h = self.re_comp(pattern, dialect, flags)
+        self.determinise(h)
+        if minimise:
+            self.minimise(h)
+        if endid is not None:
+            self.setendid(h, endid)
+        return h
+
+    def union_dfa(self, patterns, dialect: int = RE_PCRE, flags: int = 0, minimise_each: bool = True,
+                  state_limit: int = 0):
+        """The rx(1)/re(1) recipe (reference src/rx/main.c:487-566,1353,1371): per pattern
+        re_comp+determinise+minimise+setendid(index), fsm_union_array, fsm_determinise."""
+        hs = [self.compile_dfa(p, dialect, flags, minimise_each, endid=i) for i, p in enumerate(patterns)]
+        u = self.union_array(hs)
+        if state_limit:
+            res = self.determinise_limit(u, state_limit)
+            if res != 0:
+                self.free(u)
+                raise RuntimeError(f"union determinise: result {res} (1 = state limit {state_limit} reached)")
+        else:
+            self.determinise(u)
+        return u
+
+
+class Ref(_Recipes):
     """The unmodified reference, through oracle/ref_harness.c."""
 
     def __init__(self):
@@ -388,32 +424,6 @@ class Ref:
             self.libc.free(off); self.libc.free(ids)
         return f
 
-    def compile_dfa(self, pattern, dialect: int = RE_PCRE, flags: int = 0, minimise: bool = True,
-                    endid: int | None = None):
-        """re_comp -> fsm_determinise [-> fsm_minimise] [-> fsm_setendid]; returns handle."""
-        h = self.re_comp(pattern, dialect, flags)
-        self.determinise(h)
-        if minimise:
-            self.minimise(h)
-        if endid is not None:
-            self.setendid(h, endid)
-        return h
-
-    def union_dfa(self, patterns, dialect: int = RE_PCRE, flags: int = 0, minimise_each: bool = True,
-                  state_limit: int = 0):
-        """The rx(1)/re(1) recipe (reference src/rx/main.c:487-566,1353,1371): per pattern
-        re_comp+determinise+minimise+setendid(index), fsm_union_array, fsm_determinise."""
-        hs = [self.compile_dfa(p, dialect, flags, minimise_each, endid=i) for i, p in enumerate(patterns)]
-        u = self.union_array(hs)
-        if state_limit:
-            res = self.determinise_limit(u, state_limit)
-            if res != 0:
-                self.free(u)
-                raise RuntimeError(f"union determinise: result {res} (1 = state limit {state_limit} reached)")
-        else:
-            self.determinise(u)
-        return u
-
     # -- execution --------------------------------------------------------------------
     def epsilon_closure(self, h, nstates: int):
         off, to = C.c_void_p(), C.c_void_p()
@@ -437,7 +447,283 @@ class Ref:
             raise OSError(C.get_errno(), "refh_exec_batch")
         return out
 
+    def exec_batch_digest(self, h, base: np.ndarray, offsets: np.ndarray, mode: int = 1, nthreads: int = 1) -> str:
+        """records_digest of exec_batch: the answer for batches too large to record."""
+        return records_digest(self.exec_batch(h, base, offsets, mode=mode, nthreads=nthreads))
+
+    def exec_eager_batch_digest(self, h, base: np.ndarray, offsets: np.ndarray, id_of_bit: np.ndarray, mode: int = 1,
+                                nthreads: int = 1) -> str:
+        """records_digest of exec_eager_batch (records and id bitsets)."""
+        return records_digest(*self.exec_eager_batch(h, base, offsets, id_of_bit, mode=mode, nthreads=nthreads))
+
+    def numbering(self, h) -> str:
+        """numbering_digest of the automaton as it stands: its states, numbered as the reference numbers them."""
+        f = self.flatten(h)
+        return numbering_digest(f.dense_table(), f.is_end)
+
     def endids(self, h, state: int):
         buf = (C.c_uint * 4096)()
         c = self.lib.refh_endids(h, state, buf, 4096)
         return [int(buf[i]) for i in range(min(c, 4096))]
+
+
+# -- the reference's answers, recorded -----------------------------------------------------------
+#
+# Tests that compare with the reference get it from reference(): the compiled harness where it was
+# built, otherwise RecordedRef, which answers every query the suite makes from REF_CALLS, a record
+# of the harness's own answers.  An automaton is named by a hash of the calls that built it (inputs
+# included), a query by that name plus its arguments.  Batches of hundreds of thousands of records are
+# asked for as a digest (records_digest).  FSM_B200_REF=record runs the live harness and writes its
+# answers to REF_CALLS; FSM_B200_REF=replay uses the record even where the harness exists.
+
+REF_CALLS = os.path.join(ROOT, "tests", "golden", "ref_calls.json.xz")
+REF_MODE = os.environ.get("FSM_B200_REF", "")
+
+
+def replaying() -> bool:
+    """True when reference() answers from REF_CALLS rather than from the compiled harness."""
+    return REF_MODE == "replay" or (REF_MODE != "record" and not have_ref())
+
+
+def reference():
+    if REF_MODE == "record":
+        return RecordedRef(live=Ref())
+    return RecordedRef() if replaying() else Ref()
+
+
+def _key(*parts) -> str:
+    m = hashlib.sha256()
+    for p in parts:
+        if isinstance(p, FlatFsm):
+            p = (p.nstates, p.start, bool(p.hasstart), p.is_end, p.group_off, p.group_symbols, p.group_to, p.eps_off,
+                 p.eps_to, p.endid_off, p.endids, p.eager_off, p.eager_ids)
+        if isinstance(p, (np.integer, np.bool_)):
+            p = p.item()                             # numpy scalars key like the Python value they hold
+        if isinstance(p, tuple):
+            m.update(_key(*p).encode())
+        elif isinstance(p, np.ndarray):
+            m.update(f"{p.dtype.str}{p.shape}".encode() + np.ascontiguousarray(p).tobytes())
+        else:
+            m.update(repr(p).encode() if not isinstance(p, bytes) else p)
+        m.update(b"\0")
+    return m.hexdigest()[:32]
+
+
+def records_digest(records: np.ndarray, masks: np.ndarray | None = None) -> str:
+    """Digest of result records (and of the eager-output id bitsets [n, words] that go with them)."""
+    r = np.ascontiguousarray(records, dtype=RESULT_DTYPE)
+    if masks is None:
+        return _key(r)
+    return _key(r, np.ascontiguousarray(masks, dtype=np.uint64).reshape(r.shape[0], -1))
+
+
+def numbering_digest(table: np.ndarray, is_end: np.ndarray) -> str:
+    """Digest of a DFA's dense transition table [nstates, 256] and end bits, state numbering included."""
+    return _key(np.ascontiguousarray(table, dtype=np.uint32), np.asarray(is_end).astype(bool))
+
+
+def _to_json(v):
+    if isinstance(v, FlatFsm):
+        return {"fsm": [v.nstates, v.start, bool(v.hasstart)] +
+                       [None if a is None else a.reshape(-1).tolist() for a in
+                        (v.is_end, v.group_off, v.group_symbols, v.group_to, v.eps_off, v.eps_to, v.endid_off,
+                         v.endids, v.eager_off, v.eager_ids)]}
+    if isinstance(v, np.ndarray):
+        fields = v.dtype.names or (None,)
+        return {"nd": np.lib.format.dtype_to_descr(v.dtype), "shape": list(v.shape),
+                "v": [(v[f] if f else v).reshape(-1).tolist() for f in fields]}
+    if isinstance(v, bytes):
+        return {"bytes": base64.b64encode(v).decode()}
+    if isinstance(v, tuple):
+        return {"tuple": [_to_json(x) for x in v]}
+    if isinstance(v, list):
+        return [_to_json(x) for x in v]
+    if isinstance(v, (np.integer, np.bool_)):
+        return v.item()
+    assert v is None or isinstance(v, (int, bool, str)), type(v)
+    return v
+
+
+def _from_json(j):
+    if isinstance(j, list):
+        return [_from_json(x) for x in j]
+    if not isinstance(j, dict):
+        return j
+    if "fsm" in j:
+        n, start, hasstart, *a = j["fsm"]
+        return FlatFsm(n, start, hasstart, np.array(a[0], np.uint8), np.array(a[1], np.uint64),
+                       np.array(a[2], np.uint64).reshape(-1, 4), np.array(a[3], np.uint32), np.array(a[4], np.uint64),
+                       np.array(a[5], np.uint32), np.array(a[6], np.uint64), np.array(a[7], np.uint32),
+                       None if a[8] is None else np.array(a[8], np.uint64), None if a[9] is None else np.array(a[9], np.uint32))
+    if "nd" in j:
+        dt = np.lib.format.descr_to_dtype(j["nd"] if isinstance(j["nd"], str) else [tuple(d) for d in j["nd"]])
+        out = np.empty(j["shape"], dtype=dt)
+        for f, v in zip(dt.names or (None,), j["v"]):
+            (out[f] if f else out).reshape(-1)[:] = v
+        return out
+    if "bytes" in j:
+        return base64.b64decode(j["bytes"])
+    return tuple(_from_json(x) for x in j["tuple"])
+
+
+class _Handle:
+    """An automaton of RecordedRef: the hash of the calls that built it (and the live handle when recording)."""
+
+    def __init__(self, key: str, live=None):
+        self.key, self.live = key, live
+
+
+class RecordedRef(_Recipes):
+    """Ref's interface over REF_CALLS; with `live`, the compiled harness answers and REF_CALLS records it.
+    A record is made from scratch by one run of the whole suite (GPU tests included), so that it holds
+    exactly the calls the suite makes."""
+    _saved: dict | None = None
+
+    def __init__(self, live: Ref | None = None):
+        self.live = live
+        if RecordedRef._saved is None:
+            RecordedRef._saved = {}
+            if live is not None:
+                atexit.register(RecordedRef._write)
+            elif os.path.exists(REF_CALLS):
+                with lzma.open(REF_CALLS, "rt") as fh:
+                    RecordedRef._saved = json.load(fh)
+        self.calls = RecordedRef._saved
+
+    @staticmethod
+    def _write():
+        with lzma.open(REF_CALLS, "wt", preset=9 | lzma.PRESET_EXTREME) as fh:
+            json.dump(RecordedRef._saved, fh, separators=(",", ":"), sort_keys=True)
+
+    def _answer(self, key: str, ask):
+        if self.live is not None:
+            v = ask()
+            self.calls[key] = _to_json(v)
+            return v
+        if key not in self.calls:
+            raise LookupError(f"no recorded answer of the reference for this call ({key}); "
+                              f"record it with FSM_B200_REF=record where the compiled reference is built")
+        return _from_json(self.calls[key])
+
+    def _new(self, key: str, make) -> _Handle:
+        return _Handle(key, make() if self.live is not None else None)
+
+    def _mutate(self, h: _Handle, op: str, *args) -> None:
+        if self.live is not None:
+            getattr(self.live, op)(h.live, *args)
+        h.key = _key(op, h.key, *args)
+
+    # -- construction
+    def parse_file(self, path: str):
+        raise NotImplementedError("parse_file reads a file of the reference's tree: it needs the compiled reference")
+
+    def re_comp(self, pattern, dialect: int = RE_PCRE, flags: int = 0):
+        p = pattern.encode() if isinstance(pattern, str) else pattern
+        key = _key("re_comp", p, dialect, flags)
+        live = []
+
+        def ask():
+            try:
+                live.append(self.live.re_comp(p, dialect, flags))
+                return True
+            except ValueError:
+                return False
+        if not self._answer(key, ask):
+            raise ValueError(f"re_comp failed for {pattern!r}")
+        return _Handle(key, live[0] if live else None)
+
+    def from_flat(self, f: FlatFsm):
+        return self._new(_key("from_flat", f), lambda: self.live.from_flat(f))
+
+    def utf8dfa(self, lo: int = 0, hi: int = 0x10FFFF):
+        return self._new(_key("utf8dfa", lo, hi), lambda: self.live.utf8dfa(lo, hi))
+
+    def union_array(self, handles):
+        return self._new(_key("union_array", *[h.key for h in handles]),
+                         lambda: self.live.union_array([h.live for h in handles]))
+
+    def union_repeated_pattern_group(self, handles, id_base: int = 1):
+        return self._new(_key("union_repeated_pattern_group", id_base, *[h.key for h in handles]),
+                         lambda: self.live.union_repeated_pattern_group([h.live for h in handles], id_base))
+
+    def clone(self, h):
+        return self._new(h.key, lambda: self.live.clone(h.live))
+
+    def free(self, h) -> None:
+        if self.live is not None:
+            self.live.free(h.live)
+
+    # -- in-place operations
+    def determinise(self, h) -> None:
+        self._mutate(h, "determinise")
+
+    def minimise(self, h) -> None:
+        self._mutate(h, "minimise")
+
+    def setendid(self, h, i: int) -> None:
+        self._mutate(h, "setendid", i)
+
+    def remove_epsilons(self, h) -> None:
+        self._mutate(h, "remove_epsilons")
+
+    def star(self, h) -> None:
+        self._mutate(h, "star")
+
+    def eager_set(self, h, state: int, ident: int) -> None:
+        self._mutate(h, "eager_set", state, ident)
+
+    def determinise_limit(self, h, limit: int) -> int:
+        r = self._answer(_key("determinise_limit", h.key, limit), lambda: self.live.determinise_limit(h.live, limit))
+        h.key = _key("determinise_limit", h.key, limit)
+        return r
+
+    # -- queries
+    def flatten(self, h) -> FlatFsm:
+        return self._answer(_key("flatten", h.key), lambda: self.live.flatten(h.live))
+
+    def numbering(self, h) -> str:
+        return self._answer(_key("numbering", h.key), lambda: self.live.numbering(h.live))
+
+    def countstates(self, h) -> int:
+        return self._answer(_key("countstates", h.key), lambda: self.live.countstates(h.live))
+
+    def equal(self, a, b) -> bool:
+        return self._answer(_key("equal", a.key, b.key), lambda: self.live.equal(a.live, b.live))
+
+    def endids(self, h, state: int):
+        return self._answer(_key("endids", h.key, state), lambda: self.live.endids(h.live, state))
+
+    def exec(self, h, data: bytes):
+        return self._answer(_key("exec", h.key, bytes(data)), lambda: self.live.exec(h.live, data))
+
+    def exec_eager(self, h, data: bytes):
+        return self._answer(_key("exec_eager", h.key, bytes(data)), lambda: self.live.exec_eager(h.live, data))
+
+    def exec_batch(self, h, base: np.ndarray, offsets: np.ndarray, mode: int = 1, nthreads: int = 1) -> np.ndarray:
+        return self._answer(_key("exec_batch", h.key, base, offsets, mode),
+                            lambda: self.live.exec_batch(h.live, base, offsets, mode=mode, nthreads=nthreads))
+
+    def exec_batch_digest(self, h, base: np.ndarray, offsets: np.ndarray, mode: int = 1, nthreads: int = 1) -> str:
+        return self._answer(_key("exec_batch_digest", h.key, base, offsets, mode),
+                            lambda: self.live.exec_batch_digest(h.live, base, offsets, mode=mode, nthreads=nthreads))
+
+    def exec_eager_batch_digest(self, h, base: np.ndarray, offsets: np.ndarray, id_of_bit: np.ndarray, mode: int = 1,
+                                nthreads: int = 1) -> str:
+        return self._answer(_key("exec_eager_batch_digest", h.key, base, offsets, np.asarray(id_of_bit), mode),
+                            lambda: self.live.exec_eager_batch_digest(h.live, base, offsets, id_of_bit, mode=mode,
+                                                                      nthreads=nthreads))
+
+    def exec_eager_batch(self, h, base: np.ndarray, offsets: np.ndarray, id_of_bit: np.ndarray, mode: int = 1,
+                         nthreads: int = 1):
+        return self._answer(_key("exec_eager_batch", h.key, base, offsets, np.asarray(id_of_bit), mode),
+                            lambda: self.live.exec_eager_batch(h.live, base, offsets, id_of_bit, mode=mode, nthreads=nthreads))
+
+    def epsilon_closure(self, h, nstates: int):
+        return self._answer(_key("epsilon_closure", h.key, nstates), lambda: self.live.epsilon_closure(h.live, nstates))
+
+    def dfavm_bytes(self, h) -> bytes:
+        return self._answer(_key("dfavm_bytes", h.key), lambda: self.live.dfavm_bytes(h.live))
+
+    def vm_match_batch(self, h, base: np.ndarray, offsets: np.ndarray, nthreads: int = 1) -> np.ndarray:
+        return self._answer(_key("vm_match_batch", h.key, base, offsets),
+                            lambda: self.live.vm_match_batch(h.live, base, offsets, nthreads=nthreads))

@@ -12,8 +12,6 @@ import goldenio
 import reflib
 import libfsm_b200 as L
 
-pytestmark = pytest.mark.skipif(not reflib.have_ref(), reason="compiled reference not present")
-
 CASES = [c for c in goldenio.load_exec_cases(os.path.join(goldenio.GOLDEN_DIR, "golden_exec.npz")) if c["is_dfa"]]
 
 

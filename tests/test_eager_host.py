@@ -13,7 +13,6 @@ from libfsm_b200.desc import CDesc, FlatFsm
 from test_oracle_determinise import assert_isomorphic
 from test_oracle_eager import diamond, random_nfa
 
-pytestmark = pytest.mark.skipif(not reflib.have_ref(), reason="compiled reference not present")
 SO = os.path.join(reflib.REF_DIR, "libeager_host.so")
 
 

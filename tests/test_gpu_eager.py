@@ -127,11 +127,14 @@ def test_one_long_input_with_eager_outputs_is_chunked_and_exact(ref):
     _, inst = workloads.cfg3_patterns()
     base, _ = workloads.cfg3_lines_host(60000, inst, seed=33)
     h = ref.from_flat(c["fsm"])
+    cuts = (8 << 20, (3 << 20) + 17, (1 << 21) + 5)
+    wants = [ref.exec_eager_batch(h, np.ascontiguousarray(base[:cut]), np.array([0, cut], dtype=np.uint64), c["idlist"],
+                                  mode=1, nthreads=1) for cut in cuts]
+    ref.free(h)
     with L.Dfa(c["fsm"]) as dfa:
-        for cut in (8 << 20, (3 << 20) + 17, (1 << 21) + 5):
+        for cut, (want, wmasks) in zip(cuts, wants):
             data = np.ascontiguousarray(base[:cut])
             off = np.array([0, cut], dtype=np.uint64)
-            want, wmasks = ref.exec_eager_batch(h, data, off, c["idlist"], mode=1, nthreads=1)
             L.launch_count(reset=True)
             rec, masks = dfa.exec_batch_eager(data, off)
             assert L.launch_count() >= 5, "expected the chunked path"
@@ -141,7 +144,6 @@ def test_one_long_input_with_eager_outputs_is_chunked_and_exact(ref):
             assert (L.results_from_torch(drec) == want).all() and (dmasks.cpu().numpy().view(np.uint64) == wmasks).all(), cut
         # fewer ids fire on a prefix: the OR really is over the chunks walked
         assert (wmasks != 0).any()
-    ref.free(h)
 
 
 @pytest.mark.parametrize("die_at", [None, 100, 70000, 299999])

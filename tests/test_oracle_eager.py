@@ -10,8 +10,6 @@ import reflib
 from libfsm_b200.desc import FlatFsm
 from test_oracle_determinise import assert_isomorphic
 
-needs_ref = pytest.mark.skipif(not reflib.have_ref(), reason="compiled reference not present")
-
 import os  # noqa: E402
 import goldenio  # noqa: E402
 
@@ -39,7 +37,6 @@ def diamond(eager):
                               eager=eager)
 
 
-@needs_ref
 @pytest.mark.parametrize("eager,nstates", [({1: [7]}, 3), ({2: [7]}, 4), ({1: [7], 2: [7]}, 3), ({1: [7], 2: [8]}, 4),
                                            ({0: [1], 3: [2]}, 3)])
 def test_minimise_quirk_is_the_references(oracle, ref, eager, nstates):
@@ -63,7 +60,6 @@ def random_nfa(rng, n, with_eps=True):
     return FlatFsm.from_edges(n, 0, ends, edges, eps=eps, endids=endids, eager=eager)
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", range(60))
 def test_pipeline_with_eager_outputs_random(oracle, ref, seed):
     rng = np.random.default_rng(4000 + seed)
@@ -93,7 +89,6 @@ def test_pipeline_with_eager_outputs_random(oracle, ref, seed):
     ref.free(h)
 
 
-@needs_ref
 @pytest.mark.parametrize("patterns,inputs", [
     (["abc", "b+", "xyz"], [b"abc", b"zabcz", b"bbb", b"xyzabc", b"", b"q"]),
     (["^ab", "cd$", "e"], [b"ab", b"xab", b"cd", b"cdx", b"abecd", b"e"]),

@@ -1,5 +1,7 @@
-"""CPU: live differential of the oracle restatement against the compiled reference
-(oracle/_ref/libref_harness.so).  Skipped where the reference could not be built."""
+"""CPU: differential of the oracle restatement against the compiled reference
+(oracle/_ref/libref_harness.so), or against its recorded answers where it is not built."""
+import zlib
+
 import numpy as np
 import pytest
 
@@ -13,7 +15,7 @@ PATTERNS = [r"a[ -~]{7}\z", r"[0-9]+\.[0-9]+", r"^abc[0-9]+x$", r"(foo|bar)+baz"
 def test_exec_random_inputs(oracle, ref, pattern):
     h = ref.compile_dfa(pattern)
     f = ref.flatten(h)
-    rng = np.random.default_rng(abs(hash(pattern)) % (2 ** 32))
+    rng = np.random.default_rng(zlib.crc32(pattern.encode()))
     alpha = np.frombuffer(b"abcxyz0123456789.@fobarhelHELO \n\x00", dtype=np.uint8)
     strs = [alpha[rng.integers(0, len(alpha), int(rng.integers(0, 64)))].tobytes() for _ in range(2000)]
     base, off = reflib.offsets_for(strs)

@@ -5,8 +5,8 @@ way fsm_determinise does (LIFO worklist, determinise.c:118-185, over the entry o
 pairwise label-group analysis, determinise.c:898-1054 / :1056-1335 / :2331-2505).
 oracle/refnum_host.cpp compiles those same functions for the CPU; here their output is compared
 BIT-EXACTLY (no canonicalisation) with the DFAs the reference recorded in
-tests/golden/golden_determinise.npz and, when the compiled reference is present, with live
-reference runs on random NFAs.
+tests/golden/golden_determinise.npz and with the reference's runs on random NFAs: live where the
+compiled reference is built (table by table), otherwise against the digest of each DFA it recorded.
 """
 import ctypes as C
 import os
@@ -45,6 +45,17 @@ def host():
     return run
 
 
+def assert_numbering(ref, h, table: np.ndarray, end: np.ndarray, note=None) -> None:
+    """The host's DFA equals the reference's DFA behind h, state numbering included.  Against the live
+    reference the tables are compared row by row first, so that a failure names the states that differ."""
+    if isinstance(ref, reflib.Ref):
+        dfa = ref.flatten(h)
+        assert table.shape[0] == dfa.nstates, (note, table.shape[0], dfa.nstates)
+        bad = np.nonzero((table != dfa.dense_table()).any(axis=1) | (end.astype(bool) != np.asarray(dfa.is_end).astype(bool)))[0]
+        assert bad.size == 0, (note, "states numbered differently from the reference's:", bad[:10])
+    assert reflib.numbering_digest(table, end) == ref.numbering(h), (note, "state numbering differs from the reference's")
+
+
 DET_CASES = goldenio.load_det_cases(os.path.join(goldenio.GOLDEN_DIR, "golden_determinise.npz"))
 
 
@@ -71,36 +82,27 @@ def _random_nfa(rng, n, nedges, neps, nsyms):
     return FlatFsm.from_edges(n, 0, ends, edges, eps=eps)
 
 
-@pytest.mark.skipif(not reflib.have_ref(), reason="compiled reference not present")
 @pytest.mark.parametrize("seed", range(40))
 def test_numbering_matches_live_reference_random(host, seed):
     rng = np.random.default_rng(1000 + seed)
     n = int(rng.integers(2, 40))
     nfa = _random_nfa(rng, n, int(rng.integers(1, 4 * n)), int(rng.integers(0, n)), int(rng.integers(1, 9)))
-    ref = reflib.Ref()
+    ref = reflib.reference()
     h = ref.from_flat(nfa)
     ref.determinise(h)
-    dfa = ref.flatten(h)
+    assert_numbering(ref, h, *host(nfa))
     ref.free(h)
-    table, end = host(nfa)
-    assert table.shape[0] == dfa.nstates
-    assert np.array_equal(table, dfa.dense_table())
-    assert np.array_equal(end.astype(bool), np.asarray(dfa.is_end).astype(bool))
 
 
-@pytest.mark.skipif(not reflib.have_ref(), reason="compiled reference not present")
 @pytest.mark.parametrize("words,length", [(50, 12), (300, 30)])
 def test_numbering_matches_live_reference_config5_shape(host, words, length):
     from libfsm_b200 import workloads
     nfa = workloads.config5_nfa(words, length)
-    ref = reflib.Ref()
+    ref = reflib.reference()
     h = ref.from_flat(nfa)
     ref.determinise(h)
-    dfa = ref.flatten(h)
+    assert_numbering(ref, h, *host(nfa))
     ref.free(h)
-    table, end = host(nfa)
-    assert np.array_equal(table, dfa.dense_table())
-    assert np.array_equal(end.astype(bool), np.asarray(dfa.is_end).astype(bool))
 
 
 try:
@@ -110,13 +112,12 @@ except ImportError:                                   # hypothesis is optional
     _regex = None
 
 if _regex is not None:
-    @pytest.mark.skipif(not reflib.have_ref(), reason="compiled reference not present")
-    @settings(max_examples=80, deadline=None, suppress_health_check=[HealthCheck.function_scoped_fixture, HealthCheck.too_slow])
+    @settings(max_examples=80, deadline=None, derandomize=reflib.REF_MODE == "record" or reflib.replaying(), suppress_health_check=[HealthCheck.function_scoped_fixture, HealthCheck.too_slow])
     @given(patterns=st.lists(_regex, min_size=1, max_size=4))
     def test_numbering_matches_live_reference_regex_unions(host, patterns):
         """ε-heavy NFAs the way re(1)/rx(1) build them: re_comp, end ids, fsm_union_array
         (3000 examples of this strategy were run once while pinning; 80 per suite run)."""
-        ref = reflib.Ref()
+        ref = reflib.reference()
         hs = []
         try:
             for p in patterns:
@@ -133,9 +134,5 @@ if _regex is not None:
             u = hs[0]
         nfa = ref.flatten(u)
         ref.determinise(u)
-        dfa = ref.flatten(u)
+        assert_numbering(ref, u, *host(nfa), note=patterns)
         ref.free(u)
-        table, end = host(nfa)
-        assert table.shape[0] == dfa.nstates
-        assert np.array_equal(table, dfa.dense_table()), patterns
-        assert np.array_equal(end.astype(bool), np.asarray(dfa.is_end).astype(bool))
